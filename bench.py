@@ -1,8 +1,12 @@
 #!/usr/bin/env python
 """bench.py — QPs/sec (fwd+bwd) of the hot path at BASELINE.json's config C2, per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR (b200 arm): after the timed steps, rank 0 writes what the last of them returned to its caller -
+z* and the gradients of Q, p, G, h, float64 - as DIR/{z,dQ,dp,dG,dh}.npy (20.8 MB at C2). The inputs are seeded and the
+last timed step always runs on the same input copy for the same --steps, so two builds can be compared output for output.
 
 A "step" = QPFunction forward + backward over one batch of 128 random dense QPs
 (nz = nineq = 100, neq = 0, fp64; generator of prof-linear.py:64-75).  The path shards
@@ -32,6 +36,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the bench only reads the source tree (it may be read-only)
 
 import numpy as np   # noqa: E402
 import torch         # noqa: E402
@@ -298,6 +303,7 @@ def run_b200(args, rank, world, local_rank):
     e = torch.Tensor().to(dev).double()
     dl = torch.ones(B, n, dtype=torch.float64, device=dev)        # dl_dz = 1 (prof-linear.py:117)
     batches = make_batches(dev, 1000 * rank, NCOPIES)
+    eager_z = {}
 
     def step(i):
         t = batches[i % NCOPIES]
@@ -305,7 +311,12 @@ def run_b200(args, rank, world, local_rank):
             v.grad = None
         z = f(t["Q"], t["p"], t["G"], t["h"], e, e)
         z.backward(dl)
+        eager_z[i % NCOPIES] = z
         return z
+
+    def outputs(j):
+        """What the last step on input copy j returned to its caller: z* and the gradients of Q, p, G, h."""
+        return dict(z=eager_z[j], **{"d" + k: batches[j][k].grad for k in ("Q", "p", "G", "h")})
 
     settle_steps = settle(step, args.warmup, NCOPIES)
     # The step is 3 kernels behind ~0.5 ms of Python: capture QPFunction forward + autograd backward of every input
@@ -350,12 +361,19 @@ def run_b200(args, rank, world, local_rank):
             graphs.append(gph)
         torch.cuda.synchronize()
         keep.append(leaves)
-        return graphs, keep
+
+        def graph_outputs(j):
+            """outputs(j) of the replayed step: what the last replay of graph j left in its output buffers."""
+            if user_level:
+                return dict(z=keep[j][1], **{"d" + k: leaves[j][k].grad for k in ("Q", "p", "G", "h")})
+            st_, g = keep[j]
+            return dict(z=st_.zhat, dQ=g[0], dp=g[1], dG=g[2], dh=g[3])
+        return graphs, keep, graph_outputs
 
     if os.environ.get("QPB_BENCH_GRAPHS", "1") == "1":
         for user_level in (True, False):
             try:
-                graphs, keep = capture_graphs(user_level)
+                graphs, keep, outputs = capture_graphs(user_level)
 
                 def step(i):                                      # noqa: F811
                     graphs[i % NCOPIES].replay()
@@ -363,7 +381,7 @@ def run_b200(args, rank, world, local_rank):
                 launch_mode = "cuda_graph (QPFunction forward + autograd backward)" if user_level else "cuda_graph (solve_forward + solve_backward)"
                 if bench_mode != "latency":                       # the single-stream leg: one QP per SM
                     qpmod.MODE = "latency"
-                    lat_graphs, lat_keep = capture_graphs(user_level)
+                    lat_graphs, lat_keep, _ = capture_graphs(user_level)
                     qpmod.MODE = bench_mode
 
                     def serial_step(i):                           # noqa: F811
@@ -413,7 +431,9 @@ def run_b200(args, rank, world, local_rank):
         return max(e0.elapsed_time(e1) for e1 in ends)
 
     use_streams = vstreams if inflight > 1 else None
-    done = settle_steps
+    # the warm-up length depends on the allocator; starting on copy 0 keeps the input copy of every timed step (and so
+    # what --dump-outputs writes) a function of --steps alone
+    done = -(-settle_steps // NCOPIES) * NCOPIES
     timed_window(args.steps, done, use_streams)       # untimed rehearsal: same run-ahead, same allocation pattern
     done += args.steps
     timed_window(max(4, args.steps // 2), done, None)
@@ -433,6 +453,10 @@ def run_b200(args, rank, world, local_rank):
     finally:
         gc.enable()
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, v in outputs((done + args.steps - 1) % NCOPIES).items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), v.detach().to(torch.float64).cpu().numpy())
     iters_mean = float((last_iters if launch_mode.startswith("cuda_graph") else f.last_solve().iters).float().mean())
     if world > 1:
         tt = torch.tensor([ms], dtype=torch.float64, device=dev)
@@ -815,7 +839,12 @@ def main():
     ap.add_argument("--steps", type=int, default=30)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.warmup = max(args.warmup, 3)
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     # stdout of this program is ONE JSON line: everything any library prints on fd 1 meanwhile (NCCL prints its version

@@ -105,6 +105,21 @@ def sudoku_structured_problem(seed=31, B=12, n=64, e=40):
     return dict(Q=0.1 * np.eye(n), p=-rs.rand(B, n), G=-np.eye(n), h=np.zeros(n), A=A, b=A @ z0, dl=rs.randn(B, n))
 
 
+def util_results(U):
+    """What the helpers of qpth/util.py (`U`: qpth_b200.util, or the reference's module) return on fixed inputs, as
+    JSON data: batch sizes, expandParam's (shape, stride, expanded), get_sizes, bdiag."""
+    import torch
+    e, Q, q, p, h = torch.Tensor(), torch.zeros(3, 4, 4), torch.zeros(4, 4), torch.zeros(4), torch.zeros(3)
+    G, A = torch.zeros(4, 3, 5), torch.zeros(4, 2, 5)
+    out = {"extract_nBatch": [U.extract_nBatch(Q, p, G[:3, :, :4], h, e, e), U.extract_nBatch(q, p, G[0, :, :4], h, e, e)],
+           "expandParam": [], "get_sizes": list(U.get_sizes(G, A)),
+           "bdiag": U.bdiag(torch.arange(6.).view(2, 3)).tolist()}
+    for X, nd in ((Q, 3), (q, 3), (p, 2), (e, 3), (torch.tensor(1.0), 2)):
+        Y, expanded = U.expandParam(X, 3, nd)
+        out["expandParam"].append([list(Y.shape), list(Y.stride()), bool(expanded)])
+    return out
+
+
 def _testpy(tag_kw):
     def build():
         return testpy_problem(**tag_kw)

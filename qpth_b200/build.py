@@ -37,26 +37,25 @@ def build(force=False, verbose=False, extra=(), out=None):
     out = out or OUT
     if not force and out == OUT and up_to_date():
         return out
-    import hashlib
     import tempfile
-    objdir = os.path.join(tempfile.gettempdir(), "qpth_b200_obj_" + hashlib.sha1(out.encode()).hexdigest()[:10])
-    os.makedirs(objdir, exist_ok=True)
     base = [nvcc_path(), "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
             "-Xcompiler", "-fPIC"] + list(extra)
     if verbose:
         base.insert(1, "-Xptxas=-v")
-    procs, objs = [], []
-    for src, defs, tag in UNITS:
-        obj = os.path.join(objdir, tag + ".o")
-        cmd = base + defs + ["-c", "-o", obj, os.path.join(HERE, "csrc", src)]
-        if verbose:
-            print(" ".join(cmd))
-        procs.append((cmd, subprocess.Popen(cmd)))
-        objs.append(obj)
-    for cmd, pr in procs:
-        if pr.wait() != 0:
-            raise subprocess.CalledProcessError(pr.returncode, cmd)
-    subprocess.check_call([nvcc_path(), "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-o", out] + objs)
+    # objects go to a private temporary directory: a fixed name under /tmp may belong to another user of the machine
+    with tempfile.TemporaryDirectory(prefix="qpth_b200_obj_") as objdir:
+        procs, objs = [], []
+        for src, defs, tag in UNITS:
+            obj = os.path.join(objdir, tag + ".o")
+            cmd = base + defs + ["-c", "-o", obj, os.path.join(HERE, "csrc", src)]
+            if verbose:
+                print(" ".join(cmd))
+            procs.append((cmd, subprocess.Popen(cmd)))
+            objs.append(obj)
+        for cmd, rc in [(cmd, pr.wait()) for cmd, pr in procs]:      # every compiler exits before the directory goes
+            if rc != 0:
+                raise subprocess.CalledProcessError(rc, cmd)
+        subprocess.check_call([nvcc_path(), "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-o", out] + objs)
     return out
 
 

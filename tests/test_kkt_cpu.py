@@ -1,6 +1,6 @@
 """CPU checks of the host-side pieces of qpth_b200/kkt.py and qpth_b200/layers.py (no GPU): the residual of the regularised
-KKT system against a densely assembled matrix (and against the real reference when /root/reference is present), and the
-golden files the GPU tests of both modules read."""
+KKT system against a densely assembled matrix and against the real reference's outputs (tests/golden/kkt_resid_reg.npz,
+oracle/gen_golden_host.py), and the golden files the GPU tests of both modules read."""
 import os
 
 import numpy as np
@@ -39,25 +39,14 @@ def test_kkt_resid_reg_matches_dense_assembly():
     assert all(torch.equal(a, b) for a, b in zip(res, res2))
 
 
-def test_kkt_resid_reg_matches_reference_when_present():
-    from oracle import ref_runner
-    if not ref_runner.available():
-        pytest.skip("reference checkout not present (GPU box)")
-    import sys
+def test_kkt_resid_reg_matches_reference_golden(golden_dir):
+    """The reference's kkt_resid_reg (batch.py:228-241) on _problem(seed=1), inputs and outputs stored."""
     from qpth_b200 import kkt
-    saved = {k: sys.modules.get(k) for k in list(sys.modules) if k == "cvxpy" or k == "qpth" or k.startswith("qpth.")}
-    try:
-        _, rb = ref_runner.load()
-        p, eps = _problem(seed=1), 1e-7
-        ours = kkt.kkt_resid_reg(p["Q"], p["d"], p["G"], p["A"], eps, p["dx"], p["ds"], p["dz"], p["dy"], p["rx"], p["rs"], p["rz"], p["ry"])
-        ref = rb.kkt_resid_reg(p["Q"], torch.diag_embed(p["d"]), p["G"], p["A"], eps, p["dx"], p["ds"], p["dz"], p["dy"],
-                               p["rx"], p["rs"], p["rz"], p["ry"])
-        for a, b in zip(ours, ref):
-            assert float((a - b).abs().max()) < 1e-12
-    finally:                              # leave no reference modules (or the cvxpy stub) behind for the other tests
-        for k in [k for k in sys.modules if k == "cvxpy" or k == "qpth" or k.startswith("qpth.")]:
-            del sys.modules[k]
-        sys.modules.update({k: v for k, v in saved.items() if v is not None})
+    g = {k: torch.from_numpy(v) for k, v in np.load(os.path.join(golden_dir, "kkt_resid_reg.npz")).items()}
+    ours = kkt.kkt_resid_reg(g["Q"], g["d"], g["G"], g["A"], float(g["eps"]), g["dx"], g["ds"], g["dz"], g["dy"],
+                             g["rx"], g["rs"], g["rz"], g["ry"])
+    for a, k in zip(ours, ("resx", "ress", "resz", "resy")):
+        assert float((a - g[k]).abs().max()) < 1e-12
 
 
 def test_golden_files_of_the_kkt_and_layer_tests_exist(golden_dir):
