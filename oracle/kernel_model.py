@@ -83,7 +83,13 @@ def _step(v, dv):
     return 1.0 if st == np.inf else st       # every dv > 0: the fill is max(1.0, negative) = 1.0 at nBatch=1
 
 
-def solve_one(Q, p, G, h, A, b, eps=1e-12, notImprovedLim=3, maxIter=20, stall_tol=np.inf, use_eps=True, tie=1.0, noise=None):
+def solve_one(Q, p, G, h, A, b, eps=1e-12, notImprovedLim=3, maxIter=20, stall_tol=np.inf, use_eps=True, tie=1.0, noise=None,
+              trace=None):
+    """One QP with the kernels' per-QP exit rules. `trace` (a list) receives one tuple per iteration:
+    (pri, dual, mu, resid, ret_it) - the four values the kernels write to their trace buffer (pri = |rz| + |ry|,
+    dual = |L r~x|) and the index of the iterate that would be returned if the loop stopped there.
+    `best_resid` is the residual of the returned iterate, as the kernels report it: on a BEST_TIE tie that is the
+    later, tied iterate's residual, not the running minimum `min_resid` the exit tests use."""
     m, n = G.shape
     f = setup(Q, G, A)
     e = f["e"]
@@ -107,27 +113,30 @@ def solve_one(Q, p, G, h, A, b, eps=1e-12, notImprovedLim=3, maxIter=20, stall_t
             rz = Gt @ xt + s - h
             ry = At @ xt - b if e > 0 else None
             mu = abs((s * z).sum() / m)
-            resid = np.linalg.norm(rz) + (np.linalg.norm(ry) if e > 0 else 0.0) \
-                + np.linalg.norm(L @ rxt) + m * mu
+            pri = np.linalg.norm(rz) + (np.linalg.norm(ry) if e > 0 else 0.0)
+            dual = np.linalg.norm(L @ rxt)
+            resid = pri + dual + m * mu
             if noise is not None:
                 resid = resid + abs(noise.randn()) * 3e-13
             d = z / s
             L22 = _chol(f["R"] + np.diag(1.0 / d))
             if best is None:
-                best = dict(resid=resid, xt=xt.copy(), s=s.copy(), z=z.copy(),
+                best = dict(resid=resid, ret_resid=resid, xt=xt.copy(), s=s.copy(), z=z.copy(),
                             y=None if y is None else y.copy(), it=it)
                 minres = resid
                 nNot = 0
             elif resid < minres:
-                best = dict(resid=resid, xt=xt.copy(), s=s.copy(), z=z.copy(),
+                best = dict(resid=resid, ret_resid=resid, xt=xt.copy(), s=s.copy(), z=z.copy(),
                             y=None if y is None else y.copy(), it=it)
                 minres = resid
                 nNot = 0
             else:
                 nNot += 1
                 if resid < tie * minres:     # within the tie factor of the minimum: prefer the later iterate
-                    best = dict(resid=minres, xt=xt.copy(), s=s.copy(), z=z.copy(),
+                    best = dict(resid=minres, ret_resid=resid, xt=xt.copy(), s=s.copy(), z=z.copy(),
                                 y=None if y is None else y.copy(), it=it)
+            if trace is not None:
+                trace.append((pri, dual, mu, resid, best["it"]))
             if (nNot == notImprovedLim and best["resid"] < stall_tol) or (use_eps and best["resid"] < eps) or mu > 1e32:
                 break
             if not np.isfinite(resid):
@@ -145,7 +154,7 @@ def solve_one(Q, p, G, h, A, b, eps=1e-12, notImprovedLim=3, maxIter=20, stall_t
                 y = y + alpha * (dya + dyc)
     x = _tri(L, best["xt"], trans=True)
     return dict(x=x, lam=best["z"], s=best["s"], nu=best["y"], f=f, iters=iters,
-                best_resid=best["resid"], best_iter=best["it"])
+                best_resid=best["ret_resid"], min_resid=best["resid"], best_iter=best["it"])
 
 
 def backward_one(sol, dl):
@@ -169,15 +178,22 @@ def backward_one(sol, dl):
     return g
 
 
-def qp_solve(Q, p, G, h, A, b, dl=None, **opts):
-    """Batched (all inputs batched) wrapper; returns stacked outputs like pdipm_oracle.qp_solve."""
+def qp_solve(Q, p, G, h, A, b, dl=None, trace=None, **opts):
+    """Batched (all inputs batched) wrapper; returns stacked outputs like pdipm_oracle.qp_solve.
+    `trace` (a list) receives one per-QP trace list (see solve_one) per QP."""
     B = Q.shape[0]
-    sols = [solve_one(Q[i], p[i], G[i], h[i], A[i], b[i], **opts) for i in range(B)]
+    sols = []
+    for i in range(B):
+        tr = None if trace is None else []
+        sols.append(solve_one(Q[i], p[i], G[i], h[i], A[i], b[i], trace=tr, **opts))
+        if trace is not None:
+            trace.append(tr)
     out = dict(zhat=np.stack([s["x"] for s in sols]), lam=np.stack([s["lam"] for s in sols]),
                slacks=np.stack([s["s"] for s in sols]),
                nus=np.stack([s["nu"] for s in sols]) if A.shape[1] > 0 else None,
                iters=np.array([s["iters"] for s in sols]),
-               best_resids=np.array([s["best_resid"] for s in sols]))
+               best_resids=np.array([s["best_resid"] for s in sols]),
+               best_iter=np.array([s["best_iter"] for s in sols]))
     if dl is not None:
         gs = [backward_one(s, dl[i]) for i, s in enumerate(sols)]
         out["grads"] = {k: np.stack([g[k] for g in gs]) for k in gs[0]}

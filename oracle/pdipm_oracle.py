@@ -188,7 +188,8 @@ def forward(Q, p, G, h, A, b, F, eps=1e-12, verbose=0, notImprovedLim=3, maxIter
                     best["y"][I] = y[I]
                 best_iter[I] = it
             if trace is not None:
-                trace.append(dict(it=it, resids=resids.copy(), mu=mu.copy(),
+                trace.append(dict(it=it, resids=resids.copy(), mu=mu.copy(), pri=np.broadcast_to(pri_resid, (B,)).copy(),
+                                  dual=dual_resid.copy(),
                                   x=x.copy(), s=s.copy(), z=z.copy()))
             bmax = best["resids"].max()
             mumin = mu.min()

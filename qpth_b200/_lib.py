@@ -100,9 +100,9 @@ def plan_for(nz, nineq, neq, two=None):
     plan.pf3_ok, else two if plan.pf2_ok). Every (shape, two) pair has its own Plan object, so concurrent callers
     never see each other's choice. QPB200_MAXQPS=2 (development knob) caps the choice at two per SM."""
     # QPB200_PF (development / A-B knob read by qpb200_plan_init: "0" never, "1" product-form kernels wherever they fit,
-    # "2" = "1" + the two-QPs-per-SM variant by default)
+    # "2" = "1" + the two-QPs-per-SM variant by default). Every knob that changes the plan is part of the key.
     key = (nz, nineq, neq, os.environ.get("QPB200_PF"), os.environ.get("QPB200_MAXQPS"), os.environ.get("QPB200_NT512"),
-           os.environ.get("QPB200_SETUP_PF"),
+           os.environ.get("QPB200_SETUP_PF"), os.environ.get("QPB200_COOP"),
            None if two is None else bool(two))
     if key not in _plans:
         p = Plan()

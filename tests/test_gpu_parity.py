@@ -38,6 +38,7 @@ def _run(prob, requires=True, **opts):
     out["nus"] = None if st.nus is None else st.nus.cpu().numpy()
     out["iters"] = st.iters.cpu().numpy()
     out["best_resid"] = st.best_resid.cpu().numpy()
+    out["plan"] = st.plan
     if prob.get("dl") is not None and requires:
         dl = torch.tensor(np.asarray(prob["dl"]).reshape(tuple(z.shape)), dtype=torch.float64, device=DEV)
         z.backward(dl)
@@ -175,6 +176,9 @@ def test_all_solve_kernel_families_agree(family, monkeypatch):
         assert plan.pf == 1 and plan.pf2_ok == 1 and plan.pf3_ok == 1
         assert (plan.pf_two, plan.pf_three) == {"pf_one": (0, 0), "pf_two": (1, 0), "pf_three": (0, 1)}[family]
     out = _run(pr)
+    used = out["plan"]         # the plan the solve ran with (not a fresh plan_for lookup)
+    assert used.coop == (family == "r1_coop"), family
+    assert (used.pf, used.pf_two, used.pf_three) == (plan.pf, plan.pf_two, plan.pf_three), family
     ref = orc.qp_solve(pr["Q"][:16], pr["p"][:16], pr["G"][:16], pr["h"][:16], pr["A"][:16], pr["b"][:16],
                        pr["dl"][:16], per_qp=True)
     assert rel_rows(out["zhat"][:16], ref["zhat"]).max() <= ZTOL
